@@ -15,6 +15,9 @@ Other models of BASELINE.json: --model gpt2-medium | vit-l16 (tokens/s or images
 --backend nccl runs the same script on stock NCCL DDP (same-box yardstick).
 --impl reference would run the unmodified reference from baseline/_ref; it cannot be
 installed on this image (needs OpenMPI: see DESIGN.md), so it reports `unavailable`.
+--dump-outputs DIR saves the loss, gradients and weights of the last device-timed step as .npy
+files; inputs are seeded and cuDNN runs deterministic convolutions, so for the ResNet models every
+run with the same arguments computes the same values and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +33,9 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
+
+# elements kept per array by --dump-outputs: two float32 arrays of 16 MB each
+DUMP_SAMPLE = 1 << 22
 
 
 def parse_args():
@@ -52,7 +58,33 @@ def parse_args():
     p.add_argument("--no-selftest", action="store_true", help="skip the multi-rank correctness self-test (N > 1)")
     p.add_argument("--hook", default="native", choices=["native", "python"],
                    help="native: C++ comm hook on the DDP reducer (default); python: cgx_hook as in the reference")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last device-timed step of the measured arm computed to DIR/<name>.npy: "
+                        "loss.npy, grads.npy (the allreduced gradients) and params.npy (the updated weights); "
+                        f"grads and params are the same seeded sample of {DUMP_SAMPLE} elements of the "
+                        "flattened parameters when the model has more")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be >= 1")
+    return args
+
+
+def last_step_outputs(params, loss):
+    """The loss of a step, the gradients its allreduce delivered and the weights its optimizer
+    wrote, as numpy arrays; gradients and weights are flattened in parameter order and reduced to
+    the same fixed, seeded sample of DUMP_SAMPLE positions when there are more."""
+    import torch
+
+    params = list(params)
+    grads = torch.cat([p.grad.detach().reshape(-1).float() for p in params])
+    weights = torch.cat([p.detach().reshape(-1).float() for p in params])
+    n = grads.numel()
+    if n > DUMP_SAMPLE:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+        idx = idx.to(grads.device)
+        grads, weights = grads[idx], weights[idx]
+    return {"loss": loss.detach().double().reshape(1).cpu().numpy(),
+            "grads": grads.cpu().numpy(), "params": weights.cpu().numpy()}
 
 
 MODEL_DEFAULTS = {
@@ -184,7 +216,10 @@ def main():
         os.environ["CGX_STOCHASTIC_ROUNDING"] = "1"
 
     torch.manual_seed(0)
-    torch.backends.cudnn.benchmark = True
+    # same arguments, same results in every run: cuDNN picks convolution algorithms by heuristics,
+    # not by timing them (timings vary from process to process), and only deterministic ones
+    torch.backends.cudnn.benchmark = False
+    torch.backends.cudnn.deterministic = True
     torch.backends.cuda.matmul.allow_tf32 = True
     torch.backends.cudnn.allow_tf32 = True
     is_lm = args.model.startswith("gpt2")
@@ -281,14 +316,17 @@ def main():
         launches = native.stats()[1] if native is not None else 0
         return t[0].item(), t[1].item(), launches, last
 
-    def run_arm():
+    def run_arm(capture=None):
         """warm-up + (1) device-timed steps on resident inputs + (2) end-to-end steps (H2D of every
-        batch from pinned memory, D2H of every loss) with the CURRENT `ddp`."""
+        batch from pinned memory, D2H of every loss) with the CURRENT `ddp`. `capture(loss)` is
+        called between (1) and (2), while the model holds what the last step of (1) computed."""
         # W >= 3: DDP rebuilds buckets after step 1, the hook registers layers at step 3
         for i in range(warm):
             step(*resident[i % len(resident)])
         torch.cuda.synchronize()
         ms_dev, _, launches, last_loss = timed(lambda i: step(*resident[i % len(resident)]), args.steps)
+        if capture is not None:
+            capture(last_loss)
         e2e = None
         if not args.no_e2e:
             pf = CudaPrefetcher(ds, dev, channels_last=not is_lm)
@@ -331,7 +369,10 @@ def main():
 
     # ---- the product arm
     ddp = make_ddp("main")
-    ms_dev, launches, last_loss, e2e = run_arm()
+    outputs = {}
+    ms_dev, launches, last_loss, e2e = run_arm(
+        capture=(lambda loss: outputs.update(last_step_outputs(net.parameters(), loss)))
+        if args.dump_outputs and rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
 
     # ---- allreduce micro-benchmark + correctness self-test at this N (the driver only runs
@@ -389,6 +430,13 @@ def main():
             "final_loss": round(float(last_loss.detach()), 4) if last_loss is not None else None,
         }
         print(json.dumps(out), flush=True)
+        if args.dump_outputs:
+            import numpy as np
+
+            out_dir = Path(args.dump_outputs)
+            out_dir.mkdir(parents=True, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(out_dir / f"{name}.npy", arr)
     dist.destroy_process_group()
     return 0
 
